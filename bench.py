@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            this package, one process per GPU (torchrun for N > 1)
   python bench.py --impl reference --steps K --warmup W     the reference's CPU path (oracle port) on the host cores
+  python bench.py ... --dump-outputs DIR                    also write the last timed step's latents to DIR/*.npy
 
 A "step" is one sample: the latent -> latent 50-step DDIM loop (reference sample_video, motionclone_functions.py:164-167)
 at BASELINE.json configs[1]: t2v_object, 16 x 512 x 512, random-init SD1.5 + v3_sd15_mm widths, fp16. The shipped YAML
@@ -371,21 +372,22 @@ def run_own_arm(args):
         torch.cuda.synchronize()
 
     def timed(fn, n, offset):
+        """(ms of the n steps, what the last step returned)"""
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for i in range(n):
-            fn(offset + i)
+            out = fn(offset + i)
         e1.record()
         barrier()
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
         if world > 1:
             tdist.all_reduce(ms, op=tdist.ReduceOp.MAX)
-        return ms.item()
+        return ms.item(), out
 
     def step_resident(i):
         pipe.set_prompt_embeds(text_res[i])
-        pipe.sample_video(noisy_latents=resident[i], return_latents=True, add_controlnet=use_cn)
+        return pipe.sample_video(noisy_latents=resident[i], return_latents=True, add_controlnet=use_cn)
 
     out_host = torch.empty(1, 4, L, infer["height"] // 8, infer["width"] // 8, dtype=torch.float16).pin_memory()
 
@@ -395,6 +397,7 @@ def run_own_arm(args):
         out = pipe.sample_video(noisy_latents=host[i], return_latents=True, add_controlnet=use_cn)
         out_host.copy_(out, non_blocking=True)
         torch.cuda.synchronize()
+        return out_host
 
     for i in range(args.warmup):
         step_resident(i)
@@ -403,10 +406,15 @@ def run_own_arm(args):
     clocks = ClockSampler(local)
     clocks.start()
     _lib.reset_launch_count()
-    ms = timed(step_resident, args.steps, args.warmup)
+    ms, last = timed(step_resident, args.steps, args.warmup)
+    outputs = {"latents": last.float().cpu()} if args.dump_outputs else None
     launches = _lib.launch_count()
-    ms_e2e = timed(step_e2e, args.steps, args.warmup + args.steps)
+    ms_e2e, last = timed(step_e2e, args.steps, args.warmup + args.steps)
+    if outputs is not None:
+        outputs["latents_e2e"] = last.float()
     clk = clocks.finish()
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs, "" if world == 1 else f"_rank{rank}")
     # roofline leg: ONE more sample with a CUDA-event pair around every launch of this package's attention kernels (on the
     # launching stream). Kept out of the timed regions above: ~8 000 event records per sample cost ~3 % of the step.
     ops.TIMER = ops.KernelTimer()
@@ -488,6 +496,17 @@ def run_own_arm(args):
     _emit(line)
 
 
+def dump_outputs(directory: str, outputs: dict, suffix: str = "") -> None:
+    """What the timed sample_video calls returned in their last step, as float32 .npy files: `latents` from the
+    device-resident loop behind the headline value, `latents_e2e` from the host-buffer loop. The inputs are seeded, so
+    two builds run with the same arguments can be compared output for output."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    for name, t in outputs.items():
+        np.save(os.path.join(directory, f"{name}{suffix}.npy"), t.to(torch.float32).numpy())
+    log(f"[bench] outputs of the last timed step written to {directory}: {', '.join(outputs)}")
+
+
 _RESULT_FD = None
 
 
@@ -514,7 +533,13 @@ def main():
     ap.add_argument("--no-cuda-graphs", action="store_true", help="A/B: launch the no-grad UNet forwards eagerly")
     ap.add_argument("--ref-budget", type=float, default=240.0, help="seconds of CPU work for --impl reference")
     ap.add_argument("--cpu-budget", type=float, default=60.0, help="seconds of CPU work for the cpu_baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the final latents of the last timed step as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours: the reference arm extrapolates from partial steps")
     # The contract is ONE JSON line on stdout. Libraries write there too (NCCL prints its version banner on the first
     # communicator when NCCL_DEBUG=VERSION is set in the environment), so everything but the result goes to stderr: file
     # descriptor 1 is pointed at stderr for the run and the line is written to the saved descriptor at the end.

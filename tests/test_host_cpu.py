@@ -142,6 +142,21 @@ def test_bench_result_line_is_alone_on_stdout():
     assert "NCCL version x" in r.stderr and "python-level noise" in r.stderr
 
 
+def test_bench_dump_outputs_and_argument_checks(tmp_path):
+    """bench.py --dump-outputs writes each returned array as DIR/<name>.npy in float32; --steps below 1 and a dump of
+    the reference arm are refused before any work starts."""
+    import bench
+    lat = torch.randn(1, 4, 2, 8, 8).half()
+    bench.dump_outputs(str(tmp_path / "out"), {"latents": lat, "latents_e2e": lat.float() * 2}, "_rank1")
+    got = np.load(tmp_path / "out" / "latents_rank1.npy")
+    assert got.dtype == np.float32 and np.array_equal(got, lat.float().numpy())
+    assert np.load(tmp_path / "out" / "latents_e2e_rank1.npy").dtype == np.float32
+    for argv in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(tmp_path)]):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + argv, capture_output=True, text=True,
+                           timeout=300)
+        assert r.returncode == 2 and r.stdout == "", r.stderr
+
+
 def test_linear_into_residual_accumulates_in_place_only_without_grad():
     """spatial.linear_into_residual: the no-grad forwards accumulate the beta = 1 GEMM INTO the residual stream (no memcpy of
     the activation); under autograd the stream tensor is left untouched (it is saved by the LayerNorm that read it)."""
