@@ -117,7 +117,8 @@ int mc_add_noise(const void* x0, const void* noise, void* out, int64_t n, float 
  * Text cross-attention forward on tcgen05 tensor cores with TMEM accumulators (csrc/cross_attn_fwd_tc.cu):
  * O = softmax(scale * Q K^T) V per (batch, head), Q [B, Nq, H*DH] (all frames of one prompt), K, V [B, Nk <= 80, H*DH].
  * Replaces the xformers call for `attn2` (models/attention.py:193-201, :280-285 -> :535-542).
- * Strides in elements (multiples of 8); head h occupies columns [h*DH, (h+1)*DH). DH in {16, 32, 40, 64, 80, 160}.
+ * Strides in elements (multiples of 8); head h occupies columns [h*DH, (h+1)*DH).
+ * DH in {8, 16, 32, 40, 64, 80, 160}.
  */
 int mc_cross_attn_fwd(const void* q, const void* k, const void* v, void* o, int B, int Nq, int Nk, int H, int DH,
                       int64_t q_stride_b, int64_t q_stride_row, int64_t kv_stride_b, int64_t kv_stride_row,

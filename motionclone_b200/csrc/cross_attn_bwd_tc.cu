@@ -37,8 +37,7 @@ struct XBCfg {
   static constexpr int OFF_BAR = OFF_V + TKV::BYTES, SMEM = OFF_BAR + 128 + 1024;
   static constexpr int DP_COL = 80, DQ_COL = 160;  // S / dS at [0,80), dP at [80,160), dQ at [160, 160 + DHP)
   static constexpr int TCOLS = (160 + DHP <= 256) ? 256 : 512;
-  static constexpr int CTAS_TMEM = 512 / TCOLS, CTAS_SMEM = (227 * 1024) / SMEM;
-  static constexpr int CTAS_PER_SM = CTAS_TMEM < CTAS_SMEM ? CTAS_TMEM : (CTAS_SMEM < 1 ? 1 : CTAS_SMEM);
+  static constexpr int CTAS_PER_SM = ctas_per_sm(TCOLS, SMEM);
 };
 
 template <int DH>
@@ -89,37 +88,6 @@ cross_attn_bwd_dq_tc_kernel(const __grid_constant__ CUtensorMap mq128, const __g
 
   if (warp == 4) {
     if (lane == 0) {
-      auto issue_ab = [&](uint32_t d, uint32_t a0, uint32_t b0) {  // D[128 x 80] = A[128 x DH] B[80 x DH]^T, both K-major
-        const uint32_t idesc = umma_idesc_f16(kXBQ, kXBK, false, false);
-        uint32_t acc = 0;
-#pragma unroll
-        for (int p = 0; p < TQ::N64; ++p)
-#pragma unroll
-          for (int ks = 0; ks < TQ::KS64; ++ks) {
-            umma_f16(d, desc_k128(a0 + TQ::part64_off(p), ks), desc_k128(b0 + TKV::part64_off(p), ks), idesc, acc);
-            acc = 1;
-          }
-#pragma unroll
-        for (int p = 0; p < TQ::N16; ++p) {
-          umma_f16(d, desc_k32(a0 + TQ::part16_off(p)), desc_k32(b0 + TKV::part16_off(p)), idesc, acc);
-          acc = 1;
-        }
-      };
-      auto issue_dq = [&]() {  // dQ = dS K: A = dS in tensor memory (8 packed columns per k16 step), B = K MN-major
-        const uint32_t b0 = smem_u32(sK);
-        const uint32_t idesc64 = umma_idesc_f16(kXBQ, TKV::W64, false, true);
-        const uint32_t idesc16 = umma_idesc_f16(kXBQ, 16, false, true);
-#pragma unroll
-        for (int ks = 0; ks < kXBK / 16; ++ks) {
-          const uint32_t a = tmem_base + ks * 8, acc = ks > 0 ? 1u : 0u;
-#pragma unroll
-          for (int p = 0; p < TKV::N64; ++p)
-            umma_f16_ts(tmem_base + X::DQ_COL + p * 64, a, desc_mn128(b0 + TKV::part64_off(p), ks), idesc64, acc);
-#pragma unroll
-          for (int p = 0; p < TKV::N16; ++p)
-            umma_f16_ts(tmem_base + X::DQ_COL + TKV::N64 * 64 + p * 16, a, desc_mn32(b0 + TKV::part16_off(p), ks), idesc16, acc);
-        }
-      };
       auto load_q = [&](int i) {
         const int st = i % QS;
         mbar_arrive_expect_tx(q_full + st, 2 * TQ::BYTES);
@@ -133,23 +101,24 @@ cross_attn_bwd_dq_tc_kernel(const __grid_constant__ CUtensorMap mq128, const __g
       mbar_wait(bar_kv, 0);
       mbar_wait(q_full, 0);
       tc_fence_after();
-      issue_ab(tmem_base, smem_u32(sQ), smem_u32(sK));
-      issue_ab(tmem_base + X::DP_COL, smem_u32(sDO), smem_u32(sV));
+      issue_kmajor<DH, kXBQ, kXBK>(tmem_base, smem_u32(sQ), smem_u32(sK));               // S = Q K^T
+      issue_kmajor<DH, kXBQ, kXBK>(tmem_base + X::DP_COL, smem_u32(sDO), smem_u32(sV));  // dP = dO V^T
       umma_commit(sdp_full);
       for (int i = 0; i < T; ++i) {
         const uint32_t ph = i & 1;
         mbar_wait(ds_full, ph);                  // dS_i written; S_i, dP_i consumed (their MMAs - and Q_i / dO_i reads - done)
         if (i > 0) mbar_wait(dq_free, ph ^ 1);   // dQ_{i-1} copied out
         tc_fence_after();
-        issue_dq();
+        // dQ = dS K: A = dS in tensor memory, B = K MN-major
+        issue_ts_mn<DH, kXBK>(tmem_base + X::DQ_COL, [&](int ks) { return tmem_base + ks * 8; }, smem_u32(sK), false);
         umma_commit(dq_full);
         if (i + QS < T) load_q(i + QS);          // refill the stage of tile i
         if (i + 1 < T) {                         // S_{i+1}, dP_{i+1} right behind dQ_i (in-order pipe)
           const int sn = (i + 1) % QS;
           mbar_wait(q_full + sn, ((i + 1) / QS) & 1);
           tc_fence_after();
-          issue_ab(tmem_base, smem_u32(sQ + sn * TQ::BYTES), smem_u32(sK));
-          issue_ab(tmem_base + X::DP_COL, smem_u32(sDO + sn * TQ::BYTES), smem_u32(sV));
+          issue_kmajor<DH, kXBQ, kXBK>(tmem_base, smem_u32(sQ + sn * TQ::BYTES), smem_u32(sK));
+          issue_kmajor<DH, kXBQ, kXBK>(tmem_base + X::DP_COL, smem_u32(sDO + sn * TQ::BYTES), smem_u32(sV));
           umma_commit(sdp_full);
         }
       }
@@ -237,40 +206,21 @@ cross_attn_bwd_dq_tc_kernel(const __grid_constant__ CUtensorMap mq128, const __g
   }
 }
 
-struct XBMaps {
-  CUtensorMap m128, m32;
-};
-template <int DH>
-static int make_xbmaps(XBMaps& m, const void* base, int H, int rows, int B, int64_t sr, int64_t sb, int box_rows) {
-  using T = TileParts<DH>;
-  int rc = make_attn_tensor_map(&m.m128, base, DH, H, rows, B, sr, sb, 64, box_rows, true);
-  if (rc) return rc;
-  if (T::N16 > 0) rc = make_attn_tensor_map(&m.m32, base, DH, H, rows, B, sr, sb, 16, box_rows, false);
-  else m.m32 = m.m128;
-  return rc;
-}
-
 template <int DH>
 static int launch_xattn_bwd(const void* q, const void* k, const void* v, const void* d_o, XBParams prm, int64_t q_sb,
                             int64_t q_sr, int64_t kv_sb, int64_t kv_sr, int64_t do_sb, int64_t do_sr, cudaStream_t st) {
   using X = XBCfg<DH>;
-  XBMaps mq, mdo, mk, mv;
-  if (make_xbmaps<DH>(mq, q, prm.H, prm.Nq, prm.B, q_sr, q_sb, kXBQ) || make_xbmaps<DH>(mdo, d_o, prm.H, prm.Nq, prm.B, do_sr, do_sb, kXBQ) ||
-      make_xbmaps<DH>(mk, k, prm.H, prm.Nk, prm.B, kv_sr, kv_sb, kXBK) || make_xbmaps<DH>(mv, v, prm.H, prm.Nk, prm.B, kv_sr, kv_sb, kXBK))
+  OperandMaps mq, mdo, mk, mv;
+  if (make_operand_maps<DH>(mq, q, prm.H, prm.Nq, prm.B, q_sr, q_sb, kXBQ) ||
+      make_operand_maps<DH>(mdo, d_o, prm.H, prm.Nq, prm.B, do_sr, do_sb, kXBQ) ||
+      make_operand_maps<DH>(mk, k, prm.H, prm.Nk, prm.B, kv_sr, kv_sb, kXBK) ||
+      make_operand_maps<DH>(mv, v, prm.H, prm.Nk, prm.B, kv_sr, kv_sb, kXBK))
     return MC_E_CUDA;
-  const int n_tiles = (prm.Nq + kXBQ - 1) / kXBQ;
-  int64_t tasks = (int64_t)n_tiles * prm.H * prm.B;
-  int tpc = (int)(tasks / (148 * X::CTAS_PER_SM * 2));
-  tpc = tpc < 1 ? 1 : (tpc > 8 ? 8 : tpc);
-  prm.tiles_per_cta = tpc;
-  const int chunks = (n_tiles + tpc - 1) / tpc;
-  if (chunks > 65535) {
-    set_error("cross_attn_bwd_dq: too many query tiles (%d)", n_tiles);
-    return MC_E_UNSUPPORTED;
-  }
+  dim3 grid;
+  if (int e = xattn_grid("cross_attn_bwd_dq", (prm.Nq + kXBQ - 1) / kXBQ, prm.H, prm.B, X::CTAS_PER_SM, prm.tiles_per_cta, grid))
+    return e;
   auto kern = cross_attn_bwd_dq_tc_kernel<DH>;
   cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, X::SMEM);
-  dim3 grid(prm.H, chunks, prm.B);
   kern<<<grid, kXBThreads, X::SMEM, st>>>(mq.m128, mq.m32, mdo.m128, mdo.m32, mk.m128, mk.m32, mv.m128, mv.m32, prm);
   count_launch();
   return check_launch("cross_attn_bwd_dq_tc");
@@ -283,37 +233,22 @@ extern "C" int mc_cross_attn_bwd_dq(const void* q, const void* k, const void* v,
                                     int64_t kv_stride_row, int64_t do_stride_b, int64_t do_stride_row,
                                     int64_t dq_stride_b, int64_t dq_stride_row, float scale, void* stream) {
   using namespace mc;
-  if (!q || !k || !v || !d_o || !dq || B <= 0 || Nq <= 0 || Nk <= 0 || H <= 0) {
-    set_error("cross_attn_bwd_dq: null pointer or non-positive dims");
-    return MC_E_INVALID;
-  }
+  const char* entry = "cross_attn_bwd_dq";
+  if (int e = check_attn_operands(entry, {q, k, v, d_o, dq}, {B, Nq, Nk, H})) return e;
   if (Nk > kXBK) {
-    set_error("cross_attn_bwd_dq: at most %d keys (text tokens) per tile, got %d", kXBK, Nk);
+    set_error("%s: at most %d keys (text tokens) per tile, got %d", entry, kXBK, Nk);
     return MC_E_UNSUPPORTED;
   }
-  if (B > 65535 || H > 65535) {
-    set_error("cross_attn_bwd_dq: at most 65535 batches / heads");
-    return MC_E_UNSUPPORTED;
-  }
-  if ((q_stride_row | kv_stride_row | dq_stride_row | q_stride_b | kv_stride_b | dq_stride_b | do_stride_b | do_stride_row) % 8 ||
-      ((uintptr_t)q | (uintptr_t)k | (uintptr_t)v | (uintptr_t)d_o | (uintptr_t)dq) % 16) {
-    set_error("cross_attn_bwd_dq: pointers must be 16-byte aligned and strides multiples of 8 elements");
-    return MC_E_INVALID;
-  }
+  if (int e = check_attn_layout(entry, B, H, {q_stride_row, kv_stride_row, dq_stride_row, q_stride_b, kv_stride_b, dq_stride_b,
+                                              do_stride_b, do_stride_row}, {q, k, v, d_o, dq}))
+    return e;
   XBParams prm{};
   prm.dq = (__half*)dq, prm.dq_sb = dq_stride_b, prm.dq_sr = dq_stride_row;
   prm.B = B, prm.Nq = Nq, prm.Nk = Nk, prm.H = H;
   prm.scale = scale, prm.scale_log2e = scale * 1.44269504088896340736f;
   cudaStream_t st = (cudaStream_t)stream;
-#define MC_XB_CASE(D)                                                                                                    \
-  case D:                                                                                                                \
-    return launch_xattn_bwd<D>(q, k, v, d_o, prm, q_stride_b, q_stride_row, kv_stride_b, kv_stride_row, do_stride_b,    \
-                               do_stride_row, st);
-  switch (DH) {
-    MC_XB_CASE(8) MC_XB_CASE(16) MC_XB_CASE(32) MC_XB_CASE(40) MC_XB_CASE(64) MC_XB_CASE(80) MC_XB_CASE(160)
-    default: break;
-  }
-#undef MC_XB_CASE
-  set_error("cross_attn_bwd_dq: unsupported head dim %d (8, 16, 32, 40, 64, 80, 160)", DH);
-  return MC_E_UNSUPPORTED;
+  return dispatch_head_dim(entry, DH, [&](auto dh) {
+    return launch_xattn_bwd<decltype(dh)::value>(q, k, v, d_o, prm, q_stride_b, q_stride_row, kv_stride_b, kv_stride_row,
+                                                 do_stride_b, do_stride_row, st);
+  });
 }

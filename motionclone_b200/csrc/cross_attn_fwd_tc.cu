@@ -43,8 +43,7 @@ struct XFCfg {
   static constexpr int SMEM = OFF_BAR + 128 + 1024;
   static constexpr int O_COL = kXK;  // S / P at TMEM [0, 80), O at [80, 80 + DHP)
   static constexpr int TCOLS = (kXK + DHP <= 128) ? 128 : 256;
-  static constexpr int CTAS_TMEM = 512 / TCOLS, CTAS_SMEM = (227 * 1024) / SMEM;
-  static constexpr int CTAS_PER_SM = CTAS_TMEM < CTAS_SMEM ? CTAS_TMEM : (CTAS_SMEM < 1 ? 1 : CTAS_SMEM);
+  static constexpr int CTAS_PER_SM = ctas_per_sm(TCOLS, SMEM);
 };
 
 template <int DH>
@@ -94,37 +93,8 @@ cross_attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap mq128, const __grid
 
   if (warp == 4) {
     if (lane == 0) {
-      auto issue_s = [&](int stage) {  // S = Q K^T: A = Q (K-major, 128 rows), B = K (K-major, 80 rows)
-        const uint32_t a0 = smem_u32(sQ + stage * TQ::BYTES), b0 = smem_u32(sK);
-        const uint32_t idesc = umma_idesc_f16(kXQ, kXK, false, false);
-        uint32_t acc = 0;
-#pragma unroll
-        for (int p = 0; p < TQ::N64; ++p)
-#pragma unroll
-          for (int ks = 0; ks < TQ::KS64; ++ks) {
-            umma_f16(tmem_base, desc_k128(a0 + TQ::part64_off(p), ks), desc_k128(b0 + TKV::part64_off(p), ks), idesc, acc);
-            acc = 1;
-          }
-#pragma unroll
-        for (int p = 0; p < TQ::N16; ++p) {
-          umma_f16(tmem_base, desc_k32(a0 + TQ::part16_off(p)), desc_k32(b0 + TKV::part16_off(p)), idesc, acc);
-          acc = 1;
-        }
-      };
-      auto issue_pv = [&]() {  // O = P V: A = P in tensor memory (8 packed columns per k16 step), B = V MN-major
-        const uint32_t b0 = smem_u32(sV);
-        const uint32_t idesc64 = umma_idesc_f16(kXQ, TKV::W64, false, true);
-        const uint32_t idesc16 = umma_idesc_f16(kXQ, 16, false, true);
-#pragma unroll
-        for (int ks = 0; ks < kXK / 16; ++ks) {
-          const uint32_t a = tmem_base + ks * 8, acc = ks > 0 ? 1u : 0u;
-#pragma unroll
-          for (int p = 0; p < TKV::N64; ++p)
-            umma_f16_ts(tmem_base + X::O_COL + p * 64, a, desc_mn128(b0 + TKV::part64_off(p), ks), idesc64, acc);
-#pragma unroll
-          for (int p = 0; p < TKV::N16; ++p)
-            umma_f16_ts(tmem_base + X::O_COL + TKV::N64 * 64 + p * 16, a, desc_mn32(b0 + TKV::part16_off(p), ks), idesc16, acc);
-        }
+      auto issue_s = [&](int stage) {  // S = Q K^T
+        issue_kmajor<DH, kXQ, kXK>(tmem_base, smem_u32(sQ + stage * TQ::BYTES), smem_u32(sK));
       };
       mbar_arrive_expect_tx(bar_kv, 2 * TKV::BYTES);
       tma_load_tile<DH, kXK>(sK, &mk128, &mk32, bar_kv, 0, h, b);
@@ -143,7 +113,8 @@ cross_attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap mq128, const __grid
         mbar_wait(p_full, ph);                     // P_i written, S_i consumed (so S_i's MMA - and Q_i's reads - are done)
         if (i > 0) mbar_wait(o_free, ph ^ 1);      // O_{i-1} copied out
         tc_fence_after();
-        issue_pv();
+        // O = P V: A = P in tensor memory, B = V MN-major
+        issue_ts_mn<DH, kXK>(tmem_base + X::O_COL, [&](int ks) { return tmem_base + ks * 8; }, smem_u32(sV), false);
         umma_commit(o_full);
         if (i + QS < T) {                          // refill Q_i's stage with tile i + QS
           const int st = i % QS;
@@ -225,41 +196,20 @@ cross_attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap mq128, const __grid
   }
 }
 
-struct XMaps {
-  CUtensorMap m128, m32;
-};
-template <int DH>
-static int make_xmaps(XMaps& m, const void* base, int H, int rows, int B, int64_t sr, int64_t sb, int box_rows) {
-  using T = TileParts<DH>;
-  int rc = make_attn_tensor_map(&m.m128, base, DH, H, rows, B, sr, sb, 64, box_rows, true);
-  if (rc) return rc;
-  if (T::N16 > 0) rc = make_attn_tensor_map(&m.m32, base, DH, H, rows, B, sr, sb, 16, box_rows, false);
-  else m.m32 = m.m128;
-  return rc;
-}
-
 template <int DH>
 static int launch_xattn_fwd(const void* q, const void* k, const void* v, XFParams prm, int64_t q_sb, int64_t q_sr, int64_t kv_sb,
                             int64_t kv_sr, cudaStream_t st) {
   using X = XFCfg<DH>;
-  XMaps mq, mk, mv;
-  if (make_xmaps<DH>(mq, q, prm.H, prm.Nq, prm.B, q_sr, q_sb, kXQ) || make_xmaps<DH>(mk, k, prm.H, prm.Nk, prm.B, kv_sr, kv_sb, kXK) ||
-      make_xmaps<DH>(mv, v, prm.H, prm.Nk, prm.B, kv_sr, kv_sb, kXK))
+  OperandMaps mq, mk, mv;
+  if (make_operand_maps<DH>(mq, q, prm.H, prm.Nq, prm.B, q_sr, q_sb, kXQ) ||
+      make_operand_maps<DH>(mk, k, prm.H, prm.Nk, prm.B, kv_sr, kv_sb, kXK) ||
+      make_operand_maps<DH>(mv, v, prm.H, prm.Nk, prm.B, kv_sr, kv_sb, kXK))
     return MC_E_CUDA;
-  const int n_tiles = (prm.Nq + kXQ - 1) / kXQ;
-  // enough CTAs for ~2 waves of (148 SMs x resident CTAs); K / V are re-read once per CTA, so longer runs amortise them
-  int64_t tasks = (int64_t)n_tiles * prm.H * prm.B;
-  int tpc = (int)(tasks / (148 * X::CTAS_PER_SM * 2));
-  tpc = tpc < 1 ? 1 : (tpc > 8 ? 8 : tpc);
-  prm.tiles_per_cta = tpc;
-  const int chunks = (n_tiles + tpc - 1) / tpc;
-  if (chunks > 65535) {
-    set_error("cross_attn_fwd: too many query tiles (%d)", n_tiles);
-    return MC_E_UNSUPPORTED;
-  }
+  dim3 grid;
+  if (int e = xattn_grid("cross_attn_fwd", (prm.Nq + kXQ - 1) / kXQ, prm.H, prm.B, X::CTAS_PER_SM, prm.tiles_per_cta, grid))
+    return e;
   auto kern = cross_attn_fwd_tc_kernel<DH>;
   cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, X::SMEM);
-  dim3 grid(prm.H, chunks, prm.B);
   kern<<<grid, kXFThreads, X::SMEM, st>>>(mq.m128, mq.m32, mk.m128, mk.m32, mv.m128, mv.m32, prm);
   count_launch();
   return check_launch("cross_attn_fwd_tc");
@@ -271,35 +221,21 @@ extern "C" int mc_cross_attn_fwd(const void* q, const void* k, const void* v, vo
                                  int64_t q_stride_b, int64_t q_stride_row, int64_t kv_stride_b, int64_t kv_stride_row,
                                  int64_t o_stride_b, int64_t o_stride_row, float scale, void* stream) {
   using namespace mc;
-  if (!q || !k || !v || !o || B <= 0 || Nq <= 0 || Nk <= 0 || H <= 0) {
-    set_error("cross_attn_fwd: null pointer or non-positive dims");
-    return MC_E_INVALID;
-  }
+  const char* entry = "cross_attn_fwd";
+  if (int e = check_attn_operands(entry, {q, k, v, o}, {B, Nq, Nk, H})) return e;
   if (Nk > kXK) {
-    set_error("cross_attn_fwd: at most %d keys (text tokens) per tile, got %d", kXK, Nk);
+    set_error("%s: at most %d keys (text tokens) per tile, got %d", entry, kXK, Nk);
     return MC_E_UNSUPPORTED;
   }
-  if (B > 65535 || H > 65535) {
-    set_error("cross_attn_fwd: at most 65535 batches / heads");
-    return MC_E_UNSUPPORTED;
-  }
-  if ((q_stride_row | kv_stride_row | o_stride_row | q_stride_b | kv_stride_b | o_stride_b) % 8 ||
-      ((uintptr_t)q | (uintptr_t)k | (uintptr_t)v | (uintptr_t)o) % 16) {
-    set_error("cross_attn_fwd: pointers must be 16-byte aligned and strides multiples of 8 elements");
-    return MC_E_INVALID;
-  }
+  if (int e = check_attn_layout(entry, B, H, {q_stride_row, kv_stride_row, o_stride_row, q_stride_b, kv_stride_b, o_stride_b},
+                                {q, k, v, o}))
+    return e;
   XFParams prm{};
   prm.o = (__half*)o, prm.o_sb = o_stride_b, prm.o_sr = o_stride_row;
   prm.B = B, prm.Nq = Nq, prm.Nk = Nk, prm.H = H;
   prm.scale_log2e = scale * 1.44269504088896340736f;
   cudaStream_t st = (cudaStream_t)stream;
-#define MC_XF_CASE(D) \
-  case D: return launch_xattn_fwd<D>(q, k, v, prm, q_stride_b, q_stride_row, kv_stride_b, kv_stride_row, st);
-  switch (DH) {
-    MC_XF_CASE(8) MC_XF_CASE(16) MC_XF_CASE(32) MC_XF_CASE(40) MC_XF_CASE(64) MC_XF_CASE(80) MC_XF_CASE(160)
-    default: break;
-  }
-#undef MC_XF_CASE
-  set_error("cross_attn_fwd: unsupported head dim %d (8, 16, 32, 40, 64, 80, 160)", DH);
-  return MC_E_UNSUPPORTED;
+  return dispatch_head_dim(entry, DH, [&](auto dh) {
+    return launch_xattn_fwd<decltype(dh)::value>(q, k, v, prm, q_stride_b, q_stride_row, kv_stride_b, kv_stride_row, st);
+  });
 }

@@ -78,46 +78,8 @@ __global__ void __launch_bounds__(256) attn_bwd_prep_kernel(const __half* __rest
   dsc[dst] = acc * scale;
 }
 
-// D[128 x DH] (+)= A[128 x 64] B[64 x DH]: A = fp16 pairs in TENSOR MEMORY (P^T / dS / dS^T written there by the compute
-// threads; k16 step ks at a_tmem(ks)), B = a 64-row tile read MN-major
-template <int DH, typename AddrFn>
-__device__ __forceinline__ void issue_ab64_ts(uint32_t d_tmem, AddrFn a_tmem, uint32_t sB, bool accumulate) {
-  using T = TileParts<DH, kBT>;
-  const uint32_t idesc64 = umma_idesc_f16(128, T::W64, false, true);
-  const uint32_t idesc16 = umma_idesc_f16(128, 16, false, true);
-#pragma unroll
-  for (int ks = 0; ks < kBT / 16; ++ks) {
-    const uint32_t a = a_tmem(ks);
-    const uint32_t acc = (accumulate || ks > 0) ? 1u : 0u;
-#pragma unroll
-    for (int p = 0; p < T::N64; ++p) umma_f16_ts(d_tmem + p * 64, a, desc_mn128(sB + T::part64_off(p), ks), idesc64, acc);
-#pragma unroll
-    for (int p = 0; p < T::N16; ++p)
-      umma_f16_ts(d_tmem + T::N64 * 64 + p * 16, a, desc_mn32(sB + T::part16_off(p), ks), idesc16, acc);
-  }
-}
-
-// D[128 x 64] = A[128 x DH] B[64 x DH]^T: B a 64-row tile (K-major); A a 128-row tile, K-major in shared memory ...
-template <int DH>
-__device__ __forceinline__ void issue_qk64(uint32_t d_tmem, uint32_t sA, uint32_t sB) {
-  using TA = TileParts<DH, 128>;
-  using TB = TileParts<DH, kBT>;
-  const uint32_t idesc = umma_idesc_f16(128, kBT, false, false);
-  uint32_t acc = 0;
-#pragma unroll
-  for (int p = 0; p < TA::N64; ++p)
-#pragma unroll
-    for (int ks = 0; ks < TA::KS64; ++ks) {
-      umma_f16(d_tmem, desc_k128(sA + TA::part64_off(p), ks), desc_k128(sB + TB::part64_off(p), ks), idesc, acc);
-      acc = 1;
-    }
-#pragma unroll
-  for (int p = 0; p < TA::N16; ++p) {
-    umma_f16(d_tmem, desc_k32(sA + TA::part16_off(p)), desc_k32(sB + TB::part16_off(p)), idesc, acc);
-    acc = 1;
-  }
-}
-// ... or resident in tensor memory (head dims <= 48: DHP / 2 packed columns at a_tmem, see smem_row_to_tmem)
+// D[128 x 64] = A[128 x DH] B[64 x DH]^T (S, dP, S^T, dP^T) with B a 64-row tile (K-major) and A resident in tensor memory
+// (head dims <= 48: DHP / 2 packed columns at a_tmem, see smem_row_to_tmem); an A tile in shared memory takes issue_kmajor
 template <int DH>
 __device__ __forceinline__ void issue_qk64_ts(uint32_t d_tmem, uint32_t a_tmem, uint32_t sB) {
   using TB = TileParts<DH, kBT>;
@@ -145,7 +107,7 @@ struct FABwdCfg {
   static constexpr int DQ_DS = 128, DQ_ACC = 160, DQ_QT = 160 + DHP, DQ_DOT = DQ_QT + KP;
   static constexpr int DQ_NEED = AT ? DQ_DOT + KP : DQ_ACC + DHP;
   static constexpr int DQ_TCOLS = DQ_NEED <= 256 ? 256 : 512;
-  static constexpr int DQ_CTAS = (DQ_TCOLS == 256 && 2 * DQ_SMEM <= 227 * 1024) ? 2 : 1;
+  static constexpr int DQ_CTAS = ctas_per_sm(DQ_TCOLS, DQ_SMEM);
   // dKV kernel. shared memory: K, V resident; Q, dO double-buffered.
   static constexpr int KV_OFF_K = 0, KV_OFF_V = TA::BYTES, KV_OFF_Q = 2 * TA::BYTES, KV_OFF_DO = KV_OFF_Q + NS * TB::BYTES;
   // per-query statistics of the streamed tile ride the same ring: 64 x (lse2, scale D) fp32 = 512 B per stage
@@ -155,7 +117,7 @@ struct FABwdCfg {
   static constexpr int DV_COL = 128, DK_COL = 128 + DHP, KV_VT = 128 + 2 * DHP;
   static constexpr int KV_NEED = AT ? KV_VT + KP : KV_VT;
   static constexpr int KV_TCOLS = KV_NEED <= 256 ? 256 : 512;
-  static constexpr int KV_CTAS = (KV_TCOLS == 256 && 2 * KV_SMEM <= 227 * 1024) ? 2 : 1;
+  static constexpr int KV_CTAS = ctas_per_sm(KV_TCOLS, KV_SMEM);
 };
 
 // half a TMEM row (columns [c0, c0 + ncol) of DHP fp32) -> fp16 -> global
@@ -264,8 +226,8 @@ spatial_attn_bwd_dq_kernel(const __grid_constant__ CUtensorMap mq128, const __gr
           issue_qk64_ts<DH>(tmem_base, tmem_base + X::DQ_QT, smem_u32(sK + stage * TB::BYTES));
           issue_qk64_ts<DH>(tmem_base + 64, tmem_base + X::DQ_DOT, smem_u32(sV + stage * TB::BYTES));
         } else {
-          issue_qk64<DH>(tmem_base, smem_u32(sQ), smem_u32(sK + stage * TB::BYTES));
-          issue_qk64<DH>(tmem_base + 64, smem_u32(sDO), smem_u32(sV + stage * TB::BYTES));
+          issue_kmajor<DH, kBM, kBT>(tmem_base, smem_u32(sQ), smem_u32(sK + stage * TB::BYTES));
+          issue_kmajor<DH, kBM, kBT>(tmem_base + 64, smem_u32(sDO), smem_u32(sV + stage * TB::BYTES));
         }
       };
       if constexpr (X::AT) mbar_wait(a_ready, 0);
@@ -287,8 +249,8 @@ spatial_attn_bwd_dq_kernel(const __grid_constant__ CUtensorMap mq128, const __gr
         }
         mbar_wait(ds_full, ph);
         tc_fence_after();
-        issue_ab64_ts<DH>(tmem_base + X::DQ_ACC, [&](int ks) { return tmem_base + X::DQ_DS + ks * 8; },
-                          smem_u32(sK + st * TB::BYTES), j > 0);
+        issue_ts_mn<DH, kBT>(tmem_base + X::DQ_ACC, [&](int ks) { return tmem_base + X::DQ_DS + ks * 8; },
+                             smem_u32(sK + st * TB::BYTES), j > 0);
         umma_commit(dq_done);
       }
     }
@@ -425,9 +387,9 @@ spatial_attn_bwd_dkv_kernel(const __grid_constant__ CUtensorMap mk128, const __g
   } else if (warp == kBMmaWarp) {
     if (lane == 0) {
       auto issue_st = [&](int stage) {
-        issue_qk64<DH>(tmem_base, smem_u32(sK), smem_u32(sQ + stage * TB::BYTES));
+        issue_kmajor<DH, kBM, kBT>(tmem_base, smem_u32(sK), smem_u32(sQ + stage * TB::BYTES));
         if constexpr (X::AT) issue_qk64_ts<DH>(tmem_base + 64, tmem_base + X::KV_VT, smem_u32(sDO + stage * TB::BYTES));
-        else issue_qk64<DH>(tmem_base + 64, smem_u32(sV), smem_u32(sDO + stage * TB::BYTES));
+        else issue_kmajor<DH, kBM, kBT>(tmem_base + 64, smem_u32(sV), smem_u32(sDO + stage * TB::BYTES));
       };
       mbar_wait(bar_kv, 0);
       if constexpr (X::AT) mbar_wait(a_ready, 0);
@@ -440,10 +402,10 @@ spatial_attn_bwd_dkv_kernel(const __grid_constant__ CUtensorMap mk128, const __g
         const int st = i % NS;
         mbar_wait(pt_full, ph);  // P^T_i, dS^T_i in tensor memory (every thread has consumed S^T_i, dP^T_i)
         tc_fence_after();
-        issue_ab64_ts<DH>(tmem_base + X::DV_COL, [&](int ks) { return tmem_base + a_cols(ks); },
-                          smem_u32(sDO + st * TB::BYTES), i > 0);
-        issue_ab64_ts<DH>(tmem_base + X::DK_COL, [&](int ks) { return tmem_base + 64 + a_cols(ks); },
-                          smem_u32(sQ + st * TB::BYTES), i > 0);
+        issue_ts_mn<DH, kBT>(tmem_base + X::DV_COL, [&](int ks) { return tmem_base + a_cols(ks); },
+                             smem_u32(sDO + st * TB::BYTES), i > 0);
+        issue_ts_mn<DH, kBT>(tmem_base + X::DK_COL, [&](int ks) { return tmem_base + 64 + a_cols(ks); },
+                             smem_u32(sQ + st * TB::BYTES), i > 0);
         umma_commit(dkv_done);
         if (i + 1 < T_tiles) {  // next S^T, dP^T right behind (in-order pipe: P^T_i / dS^T_i are read before the overwrite)
           const int sn = (i + 1) % NS;
@@ -524,20 +486,6 @@ spatial_attn_bwd_dkv_kernel(const __grid_constant__ CUtensorMap mk128, const __g
   }
 }
 
-struct BwdMaps {
-  CUtensorMap m128, m32;
-};
-
-template <int DH>
-static int make_maps_rows(BwdMaps& m, const void* base, int H, int N, int B, int64_t sr, int64_t sb, int rows) {
-  using T = TileParts<DH>;
-  int rc = make_attn_tensor_map(&m.m128, base, DH, H, N, B, sr, sb, 64, rows, true);
-  if (rc) return rc;
-  if (T::N16 > 0) rc = make_attn_tensor_map(&m.m32, base, DH, H, N, B, sr, sb, 16, rows, false);
-  else m.m32 = m.m128;
-  return rc;
-}
-
 template <int DH>
 static int launch_spatial_bwd(const void* q, const void* k, const void* v, const void* o, const void* d_o, const float* lse,
                               float* workspace, FABwdParams prm, int64_t q_sb, int64_t q_sr, int64_t k_sb, int64_t k_sr,
@@ -545,11 +493,11 @@ static int launch_spatial_bwd(const void* q, const void* k, const void* v, const
                               cudaStream_t st) {
   using X = FABwdCfg<DH>;
   const int B = prm.B, N = prm.N, H = prm.H, Npad = prm.Npad;
-  BwdMaps q128, do128, k128, v128, q64, do64, k64, v64;
-  int rc = make_maps_rows<DH>(q128, q, H, N, B, q_sr, q_sb, 128) | make_maps_rows<DH>(do128, d_o, H, N, B, do_sr, do_sb, 128) |
-           make_maps_rows<DH>(k128, k, H, N, B, k_sr, k_sb, 128) | make_maps_rows<DH>(v128, v, H, N, B, v_sr, v_sb, 128) |
-           make_maps_rows<DH>(q64, q, H, N, B, q_sr, q_sb, kBT) | make_maps_rows<DH>(do64, d_o, H, N, B, do_sr, do_sb, kBT) |
-           make_maps_rows<DH>(k64, k, H, N, B, k_sr, k_sb, kBT) | make_maps_rows<DH>(v64, v, H, N, B, v_sr, v_sb, kBT);
+  OperandMaps q128, do128, k128, v128, q64, do64, k64, v64;
+  int rc = make_operand_maps<DH>(q128, q, H, N, B, q_sr, q_sb, kBM) | make_operand_maps<DH>(do128, d_o, H, N, B, do_sr, do_sb, kBM) |
+           make_operand_maps<DH>(k128, k, H, N, B, k_sr, k_sb, kBM) | make_operand_maps<DH>(v128, v, H, N, B, v_sr, v_sb, kBM) |
+           make_operand_maps<DH>(q64, q, H, N, B, q_sr, q_sb, kBT) | make_operand_maps<DH>(do64, d_o, H, N, B, do_sr, do_sb, kBT) |
+           make_operand_maps<DH>(k64, k, H, N, B, k_sr, k_sb, kBT) | make_operand_maps<DH>(v64, v, H, N, B, v_sr, v_sb, kBT);
   if (rc) {
     return MC_E_CUDA;
   }
@@ -597,34 +545,19 @@ extern "C" int mc_spatial_attn_bwd(const void* q, const void* k, const void* v, 
                                    int64_t o_stride_row, int64_t do_stride_b, int64_t do_stride_row, int64_t g_stride_b,
                                    int64_t g_stride_row, float scale, void* stream) {
   using namespace mc;
-  if (!q || !k || !v || !o || !d_o || !lse || !dq || !dk || !dv || !workspace || B <= 0 || N <= 0 || H <= 0) {
-    set_error("spatial_attn_bwd: null pointer or non-positive dims");
-    return MC_E_INVALID;
-  }
-  if (B > 65535 || H > 65535) {
-    set_error("spatial_attn_bwd: at most 65535 frames / heads");
-    return MC_E_UNSUPPORTED;
-  }
-  if ((q_stride_b | q_stride_row | k_stride_b | k_stride_row | v_stride_b | v_stride_row | o_stride_b | o_stride_row |
-       do_stride_b | do_stride_row | g_stride_b | g_stride_row) % 8 ||
-      ((uintptr_t)q | (uintptr_t)k | (uintptr_t)v | (uintptr_t)o | (uintptr_t)d_o | (uintptr_t)dq | (uintptr_t)dk |
-       (uintptr_t)dv | (uintptr_t)workspace) % 16) {
-    set_error("spatial_attn_bwd: pointers must be 16-byte aligned and strides multiples of 8 elements");
-    return MC_E_INVALID;
-  }
+  const char* entry = "spatial_attn_bwd";
+  if (int e = check_attn_operands(entry, {q, k, v, o, d_o, lse, dq, dk, dv, workspace}, {B, N, H})) return e;
+  if (int e = check_attn_layout(entry, B, H, {q_stride_b, q_stride_row, k_stride_b, k_stride_row, v_stride_b, v_stride_row,
+                                              o_stride_b, o_stride_row, do_stride_b, do_stride_row, g_stride_b, g_stride_row},
+                                {q, k, v, o, d_o, dq, dk, dv, workspace}))
+    return e;
   FABwdParams prm{};
   prm.dq = (__half*)dq, prm.dk = (__half*)dk, prm.dv = (__half*)dv, prm.g_sb = g_stride_b, prm.g_sr = g_stride_row;
   prm.B = B, prm.N = N, prm.H = H, prm.Npad = npad64(N), prm.scale = scale, prm.scale_log2e = scale * 1.44269504088896340736f;
   cudaStream_t st = (cudaStream_t)stream;
-#define MC_SB_CASE(D)                                                                                                      \
-  case D:                                                                                                                  \
-    return launch_spatial_bwd<D>(q, k, v, o, d_o, lse, (float*)workspace, prm, q_stride_b, q_stride_row, k_stride_b,       \
-                                 k_stride_row, v_stride_b, v_stride_row, o_stride_b, o_stride_row, do_stride_b, do_stride_row, st);
-  switch (DH) {
-    MC_SB_CASE(8) MC_SB_CASE(16) MC_SB_CASE(32) MC_SB_CASE(40) MC_SB_CASE(64) MC_SB_CASE(80) MC_SB_CASE(160)
-    default: break;
-  }
-#undef MC_SB_CASE
-  set_error("spatial_attn_bwd: unsupported head dim %d (8, 16, 32, 40, 64, 80, 160)", DH);
-  return MC_E_UNSUPPORTED;
+  return dispatch_head_dim(entry, DH, [&](auto dh) {
+    return launch_spatial_bwd<decltype(dh)::value>(q, k, v, o, d_o, lse, (float*)workspace, prm, q_stride_b, q_stride_row,
+                                                   k_stride_b, k_stride_row, v_stride_b, v_stride_row, o_stride_b,
+                                                   o_stride_row, do_stride_b, do_stride_row, st);
+  });
 }

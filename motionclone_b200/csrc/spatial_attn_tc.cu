@@ -61,50 +61,8 @@ struct FACfg {
   static constexpr int O_COL = 2 * BN;                       // S / P buffers at TMEM [0, BN), [BN, 2 BN); O at [2 BN, 2 BN + DHP)
   static constexpr int ACC_COLS = DHP;
   static constexpr int TCOLS = (O_COL + ACC_COLS <= 256) ? 256 : 512;
-  static constexpr int CTAS_TMEM = 512 / TCOLS, CTAS_SMEM = (227 * 1024) / SMEM;
-  static constexpr int CTAS_PER_SM = CTAS_TMEM < CTAS_SMEM ? CTAS_TMEM : (CTAS_SMEM < 1 ? 1 : CTAS_SMEM);
+  static constexpr int CTAS_PER_SM = ctas_per_sm(TCOLS, SMEM);
 };
-
-// S tile: A = Q (K-major, 128 rows), B = K (K-major, BN rows); one MMA per k16 step over the head dim
-template <int DH>
-__device__ __forceinline__ void issue_qk(uint32_t d_tmem, uint32_t sA, uint32_t sB) {
-  using T = TileParts<DH>;
-  using TK = typename FACfg<DH>::TK;
-  const uint32_t idesc = umma_idesc_f16(kFM, FACfg<DH>::BN, false, false);
-  uint32_t acc = 0;
-#pragma unroll
-  for (int p = 0; p < T::N64; ++p)
-#pragma unroll
-    for (int ks = 0; ks < T::KS64; ++ks) {
-      umma_f16(d_tmem, desc_k128(sA + T::part64_off(p), ks), desc_k128(sB + TK::part64_off(p), ks), idesc, acc);
-      acc = 1;
-    }
-#pragma unroll
-  for (int p = 0; p < T::N16; ++p) {
-    umma_f16(d_tmem, desc_k32(sA + T::part16_off(p)), desc_k32(sB + TK::part16_off(p)), idesc, acc);
-    acc = 1;
-  }
-}
-
-// O[128 x DH] (+)= P[128 x BN] V[BN x DH]: A = P in tensor memory (8 packed columns per k16 step), B = the V tile read
-// MN-major (its rows are the K dimension). One MMA per (k16 step, part of B).
-template <int DH>
-__device__ __forceinline__ void issue_pv(uint32_t o_tmem, uint32_t p_tmem, uint32_t sB, bool accumulate) {
-  using X = FACfg<DH>;
-  using T = typename X::TK;
-  const uint32_t idesc64 = umma_idesc_f16(kFM, T::W64, false, true);
-  const uint32_t idesc16 = umma_idesc_f16(kFM, 16, false, true);
-#pragma unroll
-  for (int ks = 0; ks < X::BN / 16; ++ks) {
-    const uint32_t a = p_tmem + ks * 8;
-    const uint32_t acc = (accumulate || ks > 0) ? 1u : 0u;
-#pragma unroll
-    for (int p = 0; p < T::N64; ++p) umma_f16_ts(o_tmem + p * 64, a, desc_mn128(sB + T::part64_off(p), ks), idesc64, acc);
-#pragma unroll
-    for (int p = 0; p < T::N16; ++p)
-      umma_f16_ts(o_tmem + T::N64 * 64 + p * 16, a, desc_mn32(sB + T::part16_off(p), ks), idesc16, acc);
-  }
-}
 
 // all lanes of the load warp: element DH of every key row of a landed V tile := 1.0 (see FACfg::PAD_SUM)
 template <int DH>
@@ -195,7 +153,7 @@ spatial_attn_fwd_kernel(const __grid_constant__ CUtensorMap mq128, const __grid_
       mbar_wait(bar_q, 0);
       mbar_wait(kv_full, 0);
       tc_fence_after();
-      issue_qk<DH>(tmem_base, smem_u32(sQ), smem_u32(sK));
+      issue_kmajor<DH, kFM, BN>(tmem_base, smem_u32(sQ), smem_u32(sK));
       umma_commit(s_full);
       for (int j = 0; j < T_tiles; ++j) {
         const int st = j % NS, buf = j & 1;
@@ -203,13 +161,14 @@ spatial_attn_fwd_kernel(const __grid_constant__ CUtensorMap mq128, const __grid_
           const int sn = (j + 1) % NS;
           mbar_wait(kv_full + sn, ((j + 1) / NS) & 1);
           tc_fence_after();
-          issue_qk<DH>(tmem_base + (buf ^ 1) * BN, smem_u32(sQ), smem_u32(sK + sn * TK::BYTES));
+          issue_kmajor<DH, kFM, BN>(tmem_base + (buf ^ 1) * BN, smem_u32(sQ), smem_u32(sK + sn * TK::BYTES));
           umma_commit(s_full + (buf ^ 1));
         }
         mbar_wait(p_full + buf, (j >> 1) & 1);  // every softmax thread has consumed S_j and written P_j
         if constexpr (X::PAD_SUM) mbar_wait(v_ready + st, (j / NS) & 1);
         tc_fence_after();
-        issue_pv<DH>(tmem_base + X::O_COL, tmem_base + buf * BN, smem_u32(sV + st * TK::BYTES), j > 0);
+        issue_ts_mn<DH, BN>(tmem_base + X::O_COL, [p = tmem_base + buf * BN](int ks) { return p + ks * 8; },
+                            smem_u32(sV + st * TK::BYTES), j > 0);
         umma_commit(pv_done);
         umma_commit(stage_free + st);
       }
@@ -328,28 +287,14 @@ spatial_attn_fwd_kernel(const __grid_constant__ CUtensorMap mq128, const __grid_
   }
 }
 
-struct AttnMaps {
-  CUtensorMap m128, m32;
-};
-
-// maps for one operand tensor (box height `rows`); the SW32 map is only encoded when the head dim has 16-wide parts
-template <int DH>
-static int make_maps(AttnMaps& m, const void* base, int H, int N, int B, int64_t sr, int64_t sb, int rows) {
-  using T = TileParts<DH>;
-  int rc = make_attn_tensor_map(&m.m128, base, DH, H, N, B, sr, sb, 64, rows, true);
-  if (rc) return rc;
-  if (T::N16 > 0) rc = make_attn_tensor_map(&m.m32, base, DH, H, N, B, sr, sb, 16, rows, false);
-  else m.m32 = m.m128;
-  return rc;
-}
-
 template <int DH>
 static int launch_spatial_fwd(const void* q, const void* k, const void* v, const FAParams& prm, int64_t q_sb, int64_t q_sr,
                               int64_t k_sb, int64_t k_sr, int64_t v_sb, int64_t v_sr, cudaStream_t st) {
   using X = FACfg<DH>;
-  AttnMaps mq, mk, mv;
-  if (make_maps<DH>(mq, q, prm.H, prm.N, prm.B, q_sr, q_sb, kFM) || make_maps<DH>(mk, k, prm.H, prm.N, prm.B, k_sr, k_sb, X::BN) ||
-      make_maps<DH>(mv, v, prm.H, prm.N, prm.B, v_sr, v_sb, X::BN)) {
+  OperandMaps mq, mk, mv;
+  if (make_operand_maps<DH>(mq, q, prm.H, prm.N, prm.B, q_sr, q_sb, kFM) ||
+      make_operand_maps<DH>(mk, k, prm.H, prm.N, prm.B, k_sr, k_sb, X::BN) ||
+      make_operand_maps<DH>(mv, v, prm.H, prm.N, prm.B, v_sr, v_sb, X::BN)) {
     return MC_E_CUDA;
   }
   auto kern = spatial_attn_fwd_kernel<DH>;
@@ -367,31 +312,18 @@ extern "C" int mc_spatial_attn_fwd(const void* q, const void* k, const void* v, 
                                    int64_t k_stride_row, int64_t v_stride_b, int64_t v_stride_row, int64_t o_stride_b,
                                    int64_t o_stride_row, float scale, void* stream) {
   using namespace mc;
-  if (!q || !k || !v || !o || B <= 0 || N <= 0 || H <= 0) {
-    set_error("spatial_attn_fwd: null pointer or non-positive dims");
-    return MC_E_INVALID;
-  }
-  if (B > 65535 || H > 65535) {
-    set_error("spatial_attn_fwd: at most 65535 frames / heads");
-    return MC_E_UNSUPPORTED;
-  }
-  if ((q_stride_b | q_stride_row | k_stride_b | k_stride_row | v_stride_b | v_stride_row | o_stride_b | o_stride_row) % 8 ||
-      ((uintptr_t)q | (uintptr_t)k | (uintptr_t)v | (uintptr_t)o) % 16) {
-    set_error("spatial_attn_fwd: pointers must be 16-byte aligned and strides multiples of 8 elements");
-    return MC_E_INVALID;
-  }
+  const char* entry = "spatial_attn_fwd";
+  if (int e = check_attn_operands(entry, {q, k, v, o}, {B, N, H})) return e;
+  if (int e = check_attn_layout(entry, B, H, {q_stride_b, q_stride_row, k_stride_b, k_stride_row, v_stride_b, v_stride_row,
+                                              o_stride_b, o_stride_row}, {q, k, v, o}))
+    return e;
   FAParams prm{};
   prm.lse = lse, prm.o = (__half*)o, prm.o_sb = o_stride_b, prm.o_sr = o_stride_row;
   prm.B = B, prm.N = N, prm.H = H;
   prm.scale_log2e = scale * 1.44269504088896340736f;
   cudaStream_t st = (cudaStream_t)stream;
-#define MC_SA_CASE(D) \
-  case D: return launch_spatial_fwd<D>(q, k, v, prm, q_stride_b, q_stride_row, k_stride_b, k_stride_row, v_stride_b, v_stride_row, st);
-  switch (DH) {
-    MC_SA_CASE(8) MC_SA_CASE(16) MC_SA_CASE(32) MC_SA_CASE(40) MC_SA_CASE(64) MC_SA_CASE(80) MC_SA_CASE(160)
-    default: break;
-  }
-#undef MC_SA_CASE
-  set_error("spatial_attn_fwd: unsupported head dim %d (8, 16, 32, 40, 64, 80, 160)", DH);
-  return MC_E_UNSUPPORTED;
+  return dispatch_head_dim(entry, DH, [&](auto dh) {
+    return launch_spatial_fwd<decltype(dh)::value>(q, k, v, prm, q_stride_b, q_stride_row, k_stride_b, k_stride_row,
+                                                   v_stride_b, v_stride_row, st);
+  });
 }

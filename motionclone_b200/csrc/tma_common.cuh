@@ -1,4 +1,6 @@
-// TMA tensor maps (cp.async.bulk.tensor, SASS UTMALDG) + swizzled UMMA shared-memory descriptors, sm_100a.
+// The tcgen05 attention layer (sm_100a): TMA tensor maps (cp.async.bulk.tensor, SASS UTMALDG), swizzled UMMA
+// shared-memory descriptors, MMA issue, TMEM loads / stores, and the host-side pieces every attention entry point shares
+// (operand maps, head-dim dispatch, argument checks).
 //
 // An attention operand tile is [128 rows][DH] fp16 (rows = tokens of one frame / head, DH contiguous in global memory).
 // In shared memory it is a sequence of PARTS along DH, each landed by ONE tensor-map load:
@@ -13,9 +15,37 @@
 #pragma once
 #include <cuda.h>
 
-#include "tc_common.cuh"
+#include <initializer_list>
+#include <type_traits>
+
+#include "mc_common.cuh"
 
 namespace mc {
+
+// ---- operand-tile geometry ----
+template <int DH, int ROWS = 128>
+struct TileParts {
+  static_assert(DH % 8 == 0, "head dim must be a multiple of 8 (16-byte rows)");
+  static_assert(ROWS % 8 == 0 && ROWS <= 256, "tile rows");
+  static constexpr int N64 = DH >= 64 ? DH / 64 : 1;   // SW128 parts
+  static constexpr int REM = DH >= 64 ? DH % 64 : 0;
+  static_assert(REM % 16 == 0, "head dims above 64 must be 64*a + 16*b");
+  static constexpr int N16 = REM / 16;                 // SW32 parts
+  static constexpr int DHP = DH >= 64 ? DH : (DH + 15) / 16 * 16;  // extent seen by the MMA (zero-padded below 64)
+  static constexpr int KS64 = DH >= 64 ? 4 : DHP / 16;             // k16 steps per SW128 part when DH is the K dim
+  static constexpr int W64 = DH >= 64 ? 64 : DHP;                  // N extent per SW128 part when DH is the N dim
+  static constexpr int P64 = ROWS * 128, P16 = ROWS * 32;          // bytes per part
+  static constexpr int BYTES = N64 * P64 + N16 * P16;
+  static constexpr int KSTEPS = N64 * KS64 + N16;
+  __host__ __device__ static constexpr int part64_off(int p) { return p * P64; }
+  __host__ __device__ static constexpr int part16_off(int p) { return N64 * P64 + p * P16; }
+};
+
+// CTAs of one kernel resident on an SM: bounded by tensor memory (512 columns) and by shared memory (227 KB)
+__host__ __device__ constexpr int ctas_per_sm(int tmem_cols, int smem_bytes) {
+  const int by_tmem = 512 / tmem_cols, by_smem = (227 * 1024) / smem_bytes;
+  return by_tmem < by_smem ? by_tmem : (by_smem < 1 ? 1 : by_smem);
+}
 
 // ---- host: tensor-map encode through the runtime's driver entry point (no link-time dependency on libcuda) ----
 typedef CUresult (*mc_encode_tiled_fn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
@@ -65,6 +95,87 @@ inline int make_attn_tensor_map(CUtensorMap* map, const void* base, int DH, int 
   return r == CUDA_SUCCESS ? 0 : (int)r;
 }
 
+// the two maps of one operand tensor (box height `box_rows`): SW128 parts and SW32 parts; the SW32 map is only encoded
+// when the head dim has 16-wide parts
+struct OperandMaps {
+  CUtensorMap m128, m32;
+};
+template <int DH>
+inline int make_operand_maps(OperandMaps& m, const void* base, int H, int rows, int frames, int64_t stride_r,
+                             int64_t stride_b, int box_rows) {
+  int rc = make_attn_tensor_map(&m.m128, base, DH, H, rows, frames, stride_r, stride_b, 64, box_rows, true);
+  if (rc) return rc;
+  if (TileParts<DH>::N16 > 0) rc = make_attn_tensor_map(&m.m32, base, DH, H, rows, frames, stride_r, stride_b, 16, box_rows, false);
+  else m.m32 = m.m128;
+  return rc;
+}
+
+// ---- host: what every attention entry point shares ----
+// The head dims the attention kernels are instantiated for (include/motionclone_b200.h and ops.ATTN_HEAD_DIMS
+// list the same set): calls f(std::integral_constant<int, DH>) and returns its status, MC_E_UNSUPPORTED for any other DH.
+template <typename F>
+inline int dispatch_head_dim(const char* entry, int DH, F&& f) {
+  switch (DH) {
+    case 8: return f(std::integral_constant<int, 8>{});
+    case 16: return f(std::integral_constant<int, 16>{});
+    case 32: return f(std::integral_constant<int, 32>{});
+    case 40: return f(std::integral_constant<int, 40>{});
+    case 64: return f(std::integral_constant<int, 64>{});
+    case 80: return f(std::integral_constant<int, 80>{});
+    case 160: return f(std::integral_constant<int, 160>{});
+    default: break;
+  }
+  set_error("%s: unsupported head dim %d (8, 16, 32, 40, 64, 80, 160)", entry, DH);
+  return MC_E_UNSUPPORTED;
+}
+
+// Argument checks, in the order the entry points apply them (checks of one kernel family go between the two calls):
+// every pointer set and every dim positive (MC_E_INVALID) ...
+inline int check_attn_operands(const char* entry, std::initializer_list<const void*> ptrs, std::initializer_list<int> dims) {
+  bool ok = true;
+  for (const void* p : ptrs) ok = ok && p != nullptr;
+  for (int d : dims) ok = ok && d > 0;
+  if (!ok) {
+    set_error("%s: null pointer or non-positive dims", entry);
+    return MC_E_INVALID;
+  }
+  return MC_OK;
+}
+// ... then B and H within the grid's y / z limit (MC_E_UNSUPPORTED), strides in multiples of 8 elements and 16-byte
+// aligned pointers (MC_E_INVALID)
+inline int check_attn_layout(const char* entry, int B, int H, std::initializer_list<int64_t> strides,
+                             std::initializer_list<const void*> ptrs) {
+  if (B > 65535 || H > 65535) {
+    set_error("%s: B and H must be at most 65535", entry);
+    return MC_E_UNSUPPORTED;
+  }
+  int64_t s_or = 0;
+  uintptr_t p_or = 0;
+  for (int64_t s : strides) s_or |= s;
+  for (const void* p : ptrs) p_or |= (uintptr_t)p;
+  if (s_or % 8 || p_or % 16) {
+    set_error("%s: pointers must be 16-byte aligned and strides multiples of 8 elements", entry);
+    return MC_E_INVALID;
+  }
+  return MC_OK;
+}
+
+// Grid (H, runs, B) of the cross-attention pair: a CTA takes a run of tiles_per_cta consecutive query tiles; enough CTAs
+// for ~2 waves of (148 SMs x resident CTAs); K / V are re-read once per CTA, so longer runs amortise them
+inline int xattn_grid(const char* entry, int n_tiles, int H, int B, int resident_ctas, int& tiles_per_cta, dim3& grid) {
+  const int64_t tasks = (int64_t)n_tiles * H * B;
+  int tpc = (int)(tasks / (148 * resident_ctas * 2));
+  tpc = tpc < 1 ? 1 : (tpc > 8 ? 8 : tpc);
+  const int runs = (n_tiles + tpc - 1) / tpc;
+  if (runs > 65535) {
+    set_error("%s: too many query tiles (%d)", entry, n_tiles);
+    return MC_E_UNSUPPORTED;
+  }
+  tiles_per_cta = tpc;
+  grid = dim3(H, runs, B);
+  return MC_OK;
+}
+
 // ---- device: tensor-map load into shared memory, completion on an mbarrier ----
 __device__ __forceinline__ void tma_load_4d(void* sdst, const CUtensorMap* map, uint64_t* bar, int c0, int c1, int c2,
                                             int c3) {
@@ -76,25 +187,6 @@ __device__ __forceinline__ void tma_load_4d(void* sdst, const CUtensorMap* map, 
 __device__ __forceinline__ void tma_prefetch_desc(const CUtensorMap* map) {
   asm volatile("prefetch.tensormap [%0];" ::"l"(map) : "memory");
 }
-
-// ---- operand-tile geometry ----
-template <int DH, int ROWS = 128>
-struct TileParts {
-  static_assert(DH % 8 == 0, "head dim must be a multiple of 8 (16-byte rows)");
-  static_assert(ROWS % 8 == 0 && ROWS <= 256, "tile rows");
-  static constexpr int N64 = DH >= 64 ? DH / 64 : 1;   // SW128 parts
-  static constexpr int REM = DH >= 64 ? DH % 64 : 0;
-  static_assert(REM % 16 == 0, "head dims above 64 must be 64*a + 16*b");
-  static constexpr int N16 = REM / 16;                 // SW32 parts
-  static constexpr int DHP = DH >= 64 ? DH : (DH + 15) / 16 * 16;  // extent seen by the MMA (zero-padded below 64)
-  static constexpr int KS64 = DH >= 64 ? 4 : DHP / 16;             // k16 steps per SW128 part when DH is the K dim
-  static constexpr int W64 = DH >= 64 ? 64 : DHP;                  // N extent per SW128 part when DH is the N dim
-  static constexpr int P64 = ROWS * 128, P16 = ROWS * 32;          // bytes per part
-  static constexpr int BYTES = N64 * P64 + N16 * P16;
-  static constexpr int KSTEPS = N64 * KS64 + N16;
-  __host__ __device__ static constexpr int part64_off(int p) { return p * P64; }
-  __host__ __device__ static constexpr int part16_off(int p) { return N64 * P64 + p * P16; }
-};
 
 // one thread: issue the loads of one [ROWS][DH] tile (rows r0.. of head h, frame b); bytes = TileParts<DH, ROWS>::BYTES.
 // The maps' box height must be ROWS.
@@ -144,6 +236,56 @@ __device__ __forceinline__ uint32_t umma_idesc_f16(int M, int N, bool a_mn, bool
   d |= (uint32_t)(N >> 3) << 17;
   d |= (uint32_t)(M >> 4) << 24;
   return d;
+}
+
+// ---- single-thread MMA issue + commit, TMEM loads, tcgen05 fences ----
+__device__ __forceinline__ void umma_f16(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accum) {
+  asm volatile(
+      "{\n"
+      ".reg .pred p;\n"
+      "setp.ne.b32 p, %4, 0;\n"
+      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n"
+      "}\n" ::"r"(d_tmem),
+      "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accum)
+      : "memory");
+}
+
+__device__ __forceinline__ void umma_commit(uint64_t* bar) {
+  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
+               : "memory");
+}
+
+__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&r)[16]) {
+  asm volatile(
+      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
+      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
+        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
+      : "r"(taddr));
+}
+__device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
+__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
+__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
+
+// D[AROWS x BROWS] (=)+= A[AROWS x DH] B[BROWS x DH]^T with both operands K-major tiles in shared memory (S = Q K^T,
+// dP = dO V^T and their transposes): one MMA per k16 step over the head dim, SW128 parts first, then SW32 parts
+template <int DH, int AROWS, int BROWS>
+__device__ __forceinline__ void issue_kmajor(uint32_t d_tmem, uint32_t sA, uint32_t sB) {
+  using TA = TileParts<DH, AROWS>;
+  using TB = TileParts<DH, BROWS>;
+  const uint32_t idesc = umma_idesc_f16(AROWS, BROWS, false, false);
+  uint32_t acc = 0;
+#pragma unroll
+  for (int p = 0; p < TA::N64; ++p)
+#pragma unroll
+    for (int ks = 0; ks < TA::KS64; ++ks) {
+      umma_f16(d_tmem, desc_k128(sA + TA::part64_off(p), ks), desc_k128(sB + TB::part64_off(p), ks), idesc, acc);
+      acc = 1;
+    }
+#pragma unroll
+  for (int p = 0; p < TA::N16; ++p) {
+    umma_f16(d_tmem, desc_k32(sA + TA::part16_off(p)), desc_k32(sB + TB::part16_off(p)), idesc, acc);
+    acc = 1;
+  }
 }
 
 // byte offset of (row r, 16-byte chunk c of 8) inside a K-major SW128 part written by threads (P, dS tiles)
@@ -209,6 +351,26 @@ __device__ __forceinline__ void umma_f16_ts(uint32_t d_tmem, uint32_t a_tmem, ui
       : "memory");
 }
 __device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
+
+// D[128 x DH] (+)= A[128 x KROWS] B[KROWS x DH] (P V, dS K, P^T dO, dS^T Q): A = fp16 pairs in TENSOR MEMORY, k16 step ks
+// at a_tmem(ks) (8 packed columns per step when contiguous); B = a KROWS-row tile read MN-major (its rows are the K
+// dimension), so it needs no transpose. One MMA per (k16 step, part of B).
+template <int DH, int KROWS, typename AddrFn>
+__device__ __forceinline__ void issue_ts_mn(uint32_t d_tmem, AddrFn a_tmem, uint32_t sB, bool accumulate) {
+  using T = TileParts<DH, KROWS>;
+  const uint32_t idesc64 = umma_idesc_f16(128, T::W64, false, true);
+  const uint32_t idesc16 = umma_idesc_f16(128, 16, false, true);
+#pragma unroll
+  for (int ks = 0; ks < KROWS / 16; ++ks) {
+    const uint32_t a = a_tmem(ks);
+    const uint32_t acc = (accumulate || ks > 0) ? 1u : 0u;
+#pragma unroll
+    for (int p = 0; p < T::N64; ++p) umma_f16_ts(d_tmem + p * 64, a, desc_mn128(sB + T::part64_off(p), ks), idesc64, acc);
+#pragma unroll
+    for (int p = 0; p < T::N16; ++p)
+      umma_f16_ts(d_tmem + T::N64 * 64 + p * 16, a, desc_mn32(sB + T::part16_off(p), ks), idesc16, acc);
+  }
+}
 
 __device__ __forceinline__ float ex2_approx(float x) {
   float y;

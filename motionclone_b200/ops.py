@@ -571,7 +571,8 @@ class CrossAttentionTC(torch.autograd.Function):
 # ----------------------------------------------------------------------------------------------------------------
 # spatial self-attention (tcgen05 + tensor-map TMA flash kernel, csrc/spatial_attn_tc.cu)
 # ----------------------------------------------------------------------------------------------------------------
-SPATIAL_ATTN_HEAD_DIMS = (8, 16, 32, 40, 64, 80, 160)
+# head dims the attention kernels are instantiated for: spatial self-attention and text cross-attention alike
+ATTN_HEAD_DIMS = (8, 16, 32, 40, 64, 80, 160)
 
 
 def _check_bnc(name: str, t: Tensor) -> None:
@@ -589,9 +590,9 @@ def spatial_attention_forward(q: Tensor, k: Tensor, v: Tensor, heads: int, scale
         if t.shape != q.shape:
             raise ValueError("q, k, v must share one shape")
     B, N, C = q.shape
-    if C % heads or (C // heads) not in SPATIAL_ATTN_HEAD_DIMS:
+    if C % heads or (C // heads) not in ATTN_HEAD_DIMS:
         raise NotImplementedError(f"spatial attention: head dim {C // heads if C % heads == 0 else '?'} not in "
-                                  f"{SPATIAL_ATTN_HEAD_DIMS}")
+                                  f"{ATTN_HEAD_DIMS}")
     o = torch.empty((B, N, C), dtype=q.dtype, device=q.device)
     lse = torch.empty((B, heads, N), dtype=torch.float32, device=q.device) if want_lse else None
     ev0 = TIMER.start() if TIMER is not None else None

@@ -27,9 +27,6 @@ from torch import nn
 from . import ops
 
 
-_XATTN_TC_HEAD_DIMS = (8, 16, 32, 40, 64, 80, 160)  # instantiations of csrc/cross_attn_{fwd,bwd}_tc.cu
-
-
 def _need_kernels(x, what: str) -> None:
     if not ops.glue_kernels_ok(x):
         raise TypeError(f"{what}: expected CUDA fp16 activations, got {x.device} {x.dtype} "
@@ -286,9 +283,9 @@ class CrossAttention(nn.Module):
             q = self.to_q(hidden_states).view(b, f * n, inner)                        # frames of one prompt share K/V
             kv = F.linear(ctx, self.fused_kv_weight())                                # [b, 77, 2C]: K | V column blocks
             k, v = kv[..., :inner], kv[..., inner:]
-            if ctx.shape[1] > 80 or dh not in _XATTN_TC_HEAD_DIMS or (torch.is_grad_enabled() and kv.requires_grad):
+            if ctx.shape[1] > 80 or dh not in ops.ATTN_HEAD_DIMS or (torch.is_grad_enabled() and kv.requires_grad):
                 raise NotImplementedError("text cross-attention kernel: <= 80 context tokens, head dim in "
-                                          f"{_XATTN_TC_HEAD_DIMS}, frozen K / V projections of a constant prompt")
+                                          f"{ops.ATTN_HEAD_DIMS}, frozen K / V projections of a constant prompt")
             # tcgen05 / TMEM kernels (csrc/cross_attn_{fwd,bwd}_tc.cu); dQ only: the text K / V carry no gradient here
             if torch.is_grad_enabled() and q.requires_grad:
                 o = ops.CrossAttentionTC.apply(q, k, v, h, self.scale)

@@ -11,7 +11,7 @@
 
 #include "tma_common.cuh"
 
-namespace mc {  // host symbols tc_common.cuh declares
+namespace mc {  // host symbols mc_common.cuh declares
 void set_error(const char*, ...) {}
 void count_launch() {}
 int check_launch(const char*) { return 0; }
